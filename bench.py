@@ -74,6 +74,30 @@ def peaks() -> dict:
     return {"hbm_gbs": 6650.0, "source": "fallback"}
 
 
+DUMP_BYTES = 60 << 20      # --dump-outputs: array data in all; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: write each tensor the timed path returned in its last step as DIR/<name>.npy, in float32 (float64
+    tensors stay float64), DUMP_BYTES at most in all.  Arrays are taken smallest first, each against an equal share of
+    what is left: one that fits is written whole with its shape, a larger one as the flattened elements at a sample of
+    indices drawn from a fixed seed and sorted, the same for every run with the same arguments, so that two builds of the
+    project can be compared output for output."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(items):
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False)
+        k = left // (len(items) - i) // a.itemsize
+        if a.size > k:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, size=k, replace=False, shuffle=False))
+            a = a.reshape(-1)[idx]
+        np.save(d / f"{name}.npy", a)
+        left -= a.nbytes
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled during the timed region."""
 
@@ -169,7 +193,11 @@ def main() -> None:
     ap.add_argument("--denoising", type=float, default=0.75, help="riffuse workload: img2img strength (0.75 -> 38 of 50 evals)")
     ap.add_argument("--clips", type=int, default=32, help="clips per GPU per step (clip workload)")
     ap.add_argument("--evals", type=int, default=50, help="scheduler steps = UNet evaluations per clip (denoising 1.0)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (B200 arm, rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 arm's timed path; the reference arm has none")
     if args.workload == "roundtrip" and args.clips == 32:
         args.clips = 16                      # BASELINE configs[4]: batch 128 on 8 GPUs
     if args.workload in ("clip", "roundtrip") and args.impl == "b200":
@@ -252,25 +280,29 @@ def main() -> None:
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
+        """milliseconds of `steps` calls of fn, and what the last call returned"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
+        out = None
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record(stream)
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if dist is not None:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     for _ in range(max(args.warmup, 3)):
         step_device()
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(step_device, args.steps)
+    ms_total, _ = timed(step_device, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"waveform": wave})      # step_device writes its result into `wave`
 
     # per-kernel CUDA-event timing of the same step (rank 0 reports)
     ms_cls = (ctypes.c_float * 3)()
@@ -287,7 +319,7 @@ def main() -> None:
 
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
 
     if rank != 0:
         if dist is not None:
@@ -621,17 +653,19 @@ def main_clip(args) -> None:
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
+        """milliseconds of `steps` calls of fn, and what the last call returned"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
+        out = None
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record(stream)
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if dist is not None:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     warm = max(args.warmup, 3)
     for _ in range(warm):
@@ -640,11 +674,13 @@ def main_clip(args) -> None:
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(step_device, args.steps)
+    ms_total, out = timed(step_device, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v for k, v in out.items() if isinstance(v, torch.Tensor)})
     step_e2e()
     e2e_steps = min(args.steps, 5)       # the e2e loop repeats the whole step with host I/O: bounded so a large --steps stays within minutes
-    ms_e2e = timed(step_e2e, e2e_steps)
+    ms_e2e, _ = timed(step_e2e, e2e_steps)
 
     # live tensor-core measurement: one eager (non-graph) step with CUDA events around every tcgen05 launch
     pipe.use_cuda_graph = False
@@ -818,17 +854,19 @@ def main_riffuse(args) -> None:
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
+        """milliseconds of `steps` calls of fn, and what the last call returned"""
         barrier()
         e0_, e1_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0_.record(stream)
+        out = None
         for _ in range(steps):
-            fn()
+            out = fn()
         e1_.record(stream)
         barrier()
         ms = torch.tensor([e0_.elapsed_time(e1_)], device=dev)
         if dist is not None:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     warm = max(args.warmup, 3)
     for _ in range(warm):
@@ -837,10 +875,12 @@ def main_riffuse(args) -> None:
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(step_device, args.steps)
+    ms_total, (image_u8, _) = timed(step_device, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"images": image_u8})
     step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     pipe.use_cuda_graph = False
     step_device()
     lib.rf_tc_profile_begin()

@@ -38,6 +38,31 @@ def test_reference_arm_other_ranks_print_nothing(monkeypatch):
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_budget_dtypes_and_fixed_sample(tmp_path, monkeypatch):
+    """--dump-outputs: small arrays whole with their shape, float32 unless float64; a large one as a sorted sample of its
+    elements, the same sample on every run; the data never exceeds the budget"""
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, str(ROOT))
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4000)
+    arrays = {"image": (torch.arange(2 * 3 * 4) % 256).to(torch.uint8).reshape(2, 3, 4),
+              "latents": torch.randn(2, 5).half(), "wave": torch.arange(5000, dtype=torch.float64)}
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays)
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").glob("*.npy")}
+    assert sorted(a) == ["image", "latents", "wave"]
+    assert a["image"].dtype == np.float32 and np.array_equal(a["image"], arrays["image"].numpy())
+    assert a["latents"].dtype == np.float32 and np.array_equal(a["latents"], arrays["latents"].float().numpy())
+    w = a["wave"]
+    assert w.dtype == np.float64 and w.ndim == 1 and 0 < w.size < 5000 and np.all(np.diff(w) > 0)   # distinct, in order
+    assert sum(x.nbytes for x in a.values()) <= 4000
+    for name, x in a.items():
+        assert np.array_equal(np.load(tmp_path / "b" / f"{name}.npy"), x)
+
+
 def test_workload_configs_and_eval_counts():
     """the img2img start-point arithmetic bench.py extrapolates with equals the reference's (riffusion_pipeline.py:358-396,
     SURVEY Appendix B: 38 evaluations at denoising 0.75, 50 at 1.0, 26 at 0.5) and the product scheduler's"""
