@@ -269,6 +269,8 @@ int rf_conv1x1_small_f16(const void* x_nchw, const void* w, const void* bias, in
  * numpy_to_pil); x fp16 NCHW (B,3,H,W) -> y uint8 NHWC (B,H,W,3).  Device-side glue between VAE decode and
  * rf_image_to_mel (SURVEY 8(f)-1). */
 int rf_vae_image_to_u8(const void* x_nchw, int B, int H, int W, uint8_t* y_nhwc, void* stream);
+/* the same with `* 255` and the round in fp32 (txt2img decode_latents: `.float()` after the fp16 clamp) */
+int rf_vae_image_to_u8_f32scale(const void* x_nchw, int B, int H, int W, uint8_t* y_nhwc, void* stream);
 /* conv_in: Conv2d(Cin<=8 -> Cout, 3x3, pad 1) reading NCHW fp16, writing NHWC; w = torch layout [Cout][Cin][3][3] */
 int rf_conv_in_f16(const void* x_nchw, const void* w, const void* bias, int B, int Cin, int H, int W, int Cout,
                    void* y_nhwc, void* stream);
@@ -289,6 +291,17 @@ int rf_slerp_f16(const void* v0, const void* v1, int B, long n, const float* d_a
 int rf_cfg_pndm_step_f16(const void* eps_pair, long n, float guidance, const void* h1, const void* h2,
                          const void* h3, const float* coef4, const void* sample, float ca, float cb,
                          void* eps_out, void* prev_sample, void* stream);
+/* Guidance combine + DPMSolverMultistepScheduler(dpmsolver++, midpoint, order 2).step in one pass, reproducing the
+ * reference's fp16 tensor-op sequence (one fp16 rounding per op, scalars at full fp32, division by alpha_s as a multiply
+ * by its fp32 reciprocal):
+ *   e = eu + g (et - eu);  m0 = (x - sigma_s e) / alpha_s;
+ *   x0_prev == NULL (first order):  prev = c_x x - c_0 m0
+ *   otherwise (second order):       prev = c_x x - c_0 m0 - c_d1 (inv_r0 (m0 - x0_prev))
+ * eps_pair = [uncond | text] (2n), sample / x0_prev / x0_out / prev_sample n fp16 each.  x0_out receives m0, the next
+ * step's history entry.  prev_sample may alias sample.  Every coefficient is an argument: the library keeps no state. */
+int rf_cfg_dpmpp_step_f16(const void* eps_pair, long n, float guidance, const void* sample, const void* x0_prev,
+                          float sigma_s, float alpha_s, float c_x, float c_0, float inv_r0, float c_d1, void* x0_out,
+                          void* prev_sample, void* stream);
 /* y = a*x + b*noise (scheduler.add_noise), optionally y = y*mask + z*(1-mask) (riffusion_pipeline.py:421-425) */
 int rf_axpby_f16(const void* x, const void* noise, float a, float b, const void* mask, const void* z, long n,
                  void* y, void* stream);

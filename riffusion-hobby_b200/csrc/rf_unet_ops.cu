@@ -584,6 +584,73 @@ __global__ void k_cfg_pndm_step(const __half* __restrict__ eps_pair, size_t n, f
     }
 }
 
+// ---------------------------------------------------------------- guidance + DPM-Solver++(2M) element-wise step
+// The reference applies DPMSolverMultistepScheduler.step to fp16 CUDA tensors with 0-dim fp32 CPU scalars: every tensor
+// op widens its fp16 operands, computes in fp32 with the scalar at full fp32 and rounds the result to fp16 once.
+// torch divides by a CPU scalar as a multiply by its fp32 reciprocal.  This reproduces that op sequence, left to right:
+//   e   = eu + g (et - eu)                                   (fp16, as k_cfg_pndm_step)
+//   m0  = (x - sigma_s * e) * (1 / alpha_s)                  convert_model_output, x0 prediction
+//   x_t = c_x * x - c_0 * m0                                 first order
+//   x_t = c_x * x - c_0 * m0 - c_d1 * (inv_r0 * (m0 - m1))   second order (midpoint), m1 = the previous step's m0
+struct DpmppCoef {
+    float g, sigma_s, inv_alpha_s, c_x, c_0, inv_r0, c_d1;
+};
+
+__device__ __forceinline__ __half rn(float v) { return __float2half_rn(v); }
+__device__ __forceinline__ float wf(__half v) { return __half2float(v); }
+
+template <bool SECOND>
+__device__ __forceinline__ void dpmpp_elem(__half eu, __half et, __half x, __half m1, const DpmppCoef& c, __half& m0_out,
+                                           __half& xt_out) {
+    const __half d = __hsub(et, eu);
+    const __half e = __hadd(eu, rn(wf(d) * c.g));
+    const __half m0 = rn(wf(rn(wf(x) - wf(rn(c.sigma_s * wf(e))))) * c.inv_alpha_s);
+    __half xt = rn(wf(rn(c.c_x * wf(x))) - wf(rn(c.c_0 * wf(m0))));
+    if constexpr (SECOND) {
+        const __half d1 = rn(c.inv_r0 * wf(rn(wf(m0) - wf(m1))));
+        xt = rn(wf(xt) - wf(rn(c.c_d1 * wf(d1))));
+    }
+    m0_out = m0;
+    xt_out = xt;
+}
+
+// n8 elements (a multiple of 8, every stream 16-byte aligned except possibly the text half of eps_pair) in 16-byte
+// groups, the remaining n - n8 < 8 one by one.  sample may alias prev_sample: each element is read before it is written
+// by the same thread.
+template <bool SECOND>
+__global__ void k_cfg_dpmpp_step(const __half* __restrict__ eps_pair, size_t n, size_t n8, bool et_vec,
+                                 const __half* sample, const __half* x0_prev, DpmppCoef c, __half* x0_out,
+                                 __half* prev_sample) {
+    const size_t tid = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    const size_t stride = static_cast<size_t>(gridDim.x) * blockDim.x;
+    const __half* et_base = eps_pair + n;
+    for (size_t gi = tid; gi < n8 / 8; gi += stride) {
+        const size_t i = gi * 8;
+        union V8 { uint4 u; __half h[8]; };
+        V8 eu, et, x, m1, m0, xt;
+        eu.u = *reinterpret_cast<const uint4*>(eps_pair + i);
+        if (et_vec) {
+            et.u = *reinterpret_cast<const uint4*>(et_base + i);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 8; ++k) et.h[k] = et_base[i + k];
+        }
+        x.u = *reinterpret_cast<const uint4*>(sample + i);
+        if constexpr (SECOND) m1.u = *reinterpret_cast<const uint4*>(x0_prev + i);
+        else m1.u = make_uint4(0, 0, 0, 0);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) dpmpp_elem<SECOND>(eu.h[k], et.h[k], x.h[k], m1.h[k], c, m0.h[k], xt.h[k]);
+        *reinterpret_cast<uint4*>(x0_out + i) = m0.u;
+        *reinterpret_cast<uint4*>(prev_sample + i) = xt.u;
+    }
+    for (size_t i = n8 + tid; i < n; i += stride) {
+        __half m0, xt;
+        dpmpp_elem<SECOND>(eps_pair[i], et_base[i], sample[i], SECOND ? x0_prev[i] : __half(), c, m0, xt);
+        x0_out[i] = m0;
+        prev_sample[i] = xt;
+    }
+}
+
 // add_noise / mask blend: y = a*x + b*n (scheduler.add_noise), optionally blended y*m + z*(1-m)
 __global__ void k_axpby(const __half* __restrict__ x, const __half* __restrict__ nz, float a, float b,
                         const __half* __restrict__ mask, const __half* __restrict__ z, size_t n,
@@ -634,6 +701,9 @@ __global__ void k_conv1x1_small(const __half* __restrict__ x, const __half* __re
 
 // VAE output -> PIL-equivalent uint8 image: (x/2 + 0.5).clamp(0,1) * 255, round half to even (numpy .round()),
 // NCHW fp16 (B,3,H,W) -> NHWC uint8 (B,H,W,3)      (riffusion_pipeline.py:430-434 + numpy_to_pil)
+// F32_SCALE: the txt2img pipeline's decode_latents, which calls `.float()` after the clamp, so `* 255` and the round
+// happen in fp32 instead of fp16.
+template <bool F32_SCALE>
 __global__ void k_vae_to_u8(const __half* __restrict__ x, int B, size_t HW, uint8_t* __restrict__ y) {
     const size_t n = static_cast<size_t>(B) * HW;
     for (size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
@@ -646,7 +716,10 @@ __global__ void k_vae_to_u8(const __half* __restrict__ x, int B, size_t HW, uint
             // is float16 arithmetic too (product rounded to fp16, then round-half-even) -> the same ops in __half here
             const __half h = __hadd(__hmul(x[(b * 3 + c) * HW + p], __float2half(0.5f)), __float2half(0.5f));
             const __half cl = __hmin(__hmax(h, __float2half(0.f)), __float2half(1.f));
-            y[i * 3 + c] = static_cast<uint8_t>(__half2int_rn(hrint(__hmul(cl, __float2half(255.f)))));
+            if constexpr (F32_SCALE)
+                y[i * 3 + c] = static_cast<uint8_t>(__float2int_rn(__half2float(cl) * 255.f));
+            else
+                y[i * 3 + c] = static_cast<uint8_t>(__half2int_rn(hrint(__hmul(cl, __float2half(255.f)))));
         }
     }
 }
@@ -856,9 +929,19 @@ extern "C" int rf_conv1x1_small_f16(const void* x_nchw, const void* w, const voi
 extern "C" int rf_vae_image_to_u8(const void* x_nchw, int B, int H, int W, uint8_t* y_nhwc, void* stream) {
     if (!x_nchw || !y_nhwc || B <= 0 || H <= 0 || W <= 0) return rf_fail(RF_ERR_INVALID, "rf_vae_image_to_u8: bad argument");
     const size_t HW = static_cast<size_t>(H) * W;
-    k_vae_to_u8<<<grid_for(static_cast<size_t>(B) * HW, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+    k_vae_to_u8<false><<<grid_for(static_cast<size_t>(B) * HW, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         static_cast<const __half*>(x_nchw), B, HW, y_nhwc);
     RF_CUDA_LAUNCH_CHECK("k_vae_to_u8");
+    return RF_OK;
+}
+
+extern "C" int rf_vae_image_to_u8_f32scale(const void* x_nchw, int B, int H, int W, uint8_t* y_nhwc, void* stream) {
+    if (!x_nchw || !y_nhwc || B <= 0 || H <= 0 || W <= 0)
+        return rf_fail(RF_ERR_INVALID, "rf_vae_image_to_u8_f32scale: bad argument");
+    const size_t HW = static_cast<size_t>(H) * W;
+    k_vae_to_u8<true><<<grid_for(static_cast<size_t>(B) * HW, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        static_cast<const __half*>(x_nchw), B, HW, y_nhwc);
+    RF_CUDA_LAUNCH_CHECK("k_vae_to_u8_f32scale");
     return RF_OK;
 }
 
@@ -956,6 +1039,31 @@ extern "C" int rf_cfg_pndm_step_f16(const void* eps_pair, long n, float guidance
         static_cast<const __half*>(h2), static_cast<const __half*>(h3), coef4[0], coef4[1], coef4[2], coef4[3],
         static_cast<const __half*>(sample), ca, cb, static_cast<__half*>(eps_out), static_cast<__half*>(prev_sample));
     RF_CUDA_LAUNCH_CHECK("k_cfg_pndm_step");
+    return RF_OK;
+}
+
+extern "C" int rf_cfg_dpmpp_step_f16(const void* eps_pair, long n, float guidance, const void* sample, const void* x0_prev,
+                                     float sigma_s, float alpha_s, float c_x, float c_0, float inv_r0, float c_d1,
+                                     void* x0_out, void* prev_sample, void* stream) {
+    if (!eps_pair || !sample || !x0_out || !prev_sample || n <= 0 || !(alpha_s > 0.f) || x0_out == prev_sample)
+        return rf_fail(RF_ERR_INVALID, "rf_cfg_dpmpp_step_f16: bad argument");
+    const size_t N = static_cast<size_t>(n);
+    const auto a16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+    const bool vec = a16(eps_pair) && a16(sample) && (!x0_prev || a16(x0_prev)) && a16(x0_out) && a16(prev_sample);
+    const size_t n8 = vec ? (N & ~static_cast<size_t>(7)) : 0;
+    const bool et_vec = (N & 7) == 0;
+    const DpmppCoef c{guidance, sigma_s, 1.f / alpha_s, c_x, c_0, inv_r0, c_d1};
+    const unsigned grid = grid_for(n8 / 8 + (N - n8), 256);
+    const auto* ep = static_cast<const __half*>(eps_pair);
+    const auto* xs = static_cast<const __half*>(sample);
+    const auto* m1 = static_cast<const __half*>(x0_prev);
+    auto* m0 = static_cast<__half*>(x0_out);
+    auto* xt = static_cast<__half*>(prev_sample);
+    if (x0_prev)
+        k_cfg_dpmpp_step<true><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(ep, N, n8, et_vec, xs, m1, c, m0, xt);
+    else
+        k_cfg_dpmpp_step<false><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(ep, N, n8, et_vec, xs, m1, c, m0, xt);
+    RF_CUDA_LAUNCH_CHECK("k_cfg_dpmpp_step");
     return RF_OK;
 }
 

@@ -111,6 +111,7 @@ SIGNATURES = {
     "rf_conv1x1_small_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_long, C.c_float,
                                        C.c_void_p, C.c_void_p]),
     "rf_vae_image_to_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "rf_vae_image_to_u8_f32scale": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "rf_conv_in_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                  C.c_void_p, C.c_void_p]),
     "rf_conv_out_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
@@ -122,7 +123,9 @@ SIGNATURES = {
     "rf_cfg_pndm_step_f16": (C.c_int, [C.c_void_p, C.c_long, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_void_p, C.c_void_p,
                                        C.c_void_p]),
-    "rf_axpby_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_long,
+    "rf_cfg_dpmpp_step_f16": (C.c_int, [C.c_void_p, C.c_long, C.c_float, C.c_void_p, C.c_void_p, C.c_float, C.c_float,
+                                        C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rf_axpby_f16":(C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_long,
                                C.c_void_p, C.c_void_p]),
     "rf_attention_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.c_int, C.c_int, C.c_float, C.c_void_p]),

@@ -183,11 +183,13 @@ def _str2bool(v: str) -> bool:
     raise argparse.ArgumentTypeError(f"expected a boolean, got {v!r}")
 
 
-def build_parser() -> argparse.ArgumentParser:
-    """argh-style front end: one sub-command per function (underscores -> dashes), one --flag per keyword-only arg."""
-    parser = argparse.ArgumentParser(prog="riffusion.cli", description=__doc__)
+def build_parser(commands: T.Optional[T.Sequence[T.Callable]] = None, prog: str = "riffusion.cli",
+                 description: T.Optional[str] = __doc__) -> argparse.ArgumentParser:
+    """argh-style front end: one sub-command per function (underscores -> dashes), one --flag per keyword-only arg.
+    `commands` defaults to this module's six commands."""
+    parser = argparse.ArgumentParser(prog=prog, description=description)
     sub = parser.add_subparsers(dest="command", required=True)
-    for fn in COMMANDS:
+    for fn in (COMMANDS if commands is None else commands):
         sp = sub.add_parser(fn.__name__.replace("_", "-"), help=(fn.__doc__ or "").strip())
         sp.set_defaults(_fn=fn)
         for name, prm in inspect.signature(fn).parameters.items():

@@ -268,18 +268,7 @@ class RiffusionPipeline:
         t_start = max(num_inference_steps - init_timestep + offset, 0)                             # :392
         timesteps = self.scheduler.timesteps[t_start:]
         ctx_cache: T.Dict[str, T.Any] = {}
-        graphed = None
-        if self.use_cuda_graph and do_cfg:
-            from riffusion.graphed import GraphedUNet
-
-            # one captured graph per (latent shape, context shape); a new request only refreshes the cross-attention
-            # K / V^T that the graph reads (capture costs two eager evaluations + instantiation)
-            gkey = (tuple(latents.shape), tuple(context.shape))
-            graphed = self._graphs.get(gkey)
-            if graphed is None:
-                graphed = self._graphs[gkey] = GraphedUNet(self.unet, latents.shape, context)
-            else:
-                graphed.set_context(context)
+        graphed = self._graphed_unet(latents.shape, context) if self.use_cuda_graph and do_cfg else None
         n_evals = 0
         for t in timesteps:                                                                        # :398
             t_int = int(t)
@@ -313,6 +302,150 @@ class RiffusionPipeline:
             out["images"] = (image / 2 + 0.5).clamp(0, 1).cpu().permute(0, 2, 3, 1).numpy()         # float16 array, like the reference
         return out
 
+    def _graphed_unet(self, latent_shape, context: torch.Tensor):
+        """One captured CFG evaluation per (latent shape, context shape); a new request only refreshes the
+        cross-attention K / V^T that the graph reads (capture costs two eager evaluations + instantiation)."""
+        from riffusion.graphed import GraphedUNet
+
+        gkey = (tuple(latent_shape), tuple(context.shape))
+        graphed = self._graphs.get(gkey)
+        if graphed is None:
+            graphed = self._graphs[gkey] = GraphedUNet(self.unet, latent_shape, context)
+        else:
+            graphed.set_context(context)
+        return graphed
+
+    # ------------------------------------------------------------------------------ txt2img
+    @torch.no_grad()
+    def txt2img(self, prompt: T.Union[str, T.Sequence[str], None] = None, *,
+                negative_prompt: T.Union[str, T.Sequence[T.Optional[str]], None] = None,
+                seed: T.Union[int, T.Sequence[int]] = 42, num_inference_steps: int = 50, guidance_scale: float = 7.5,
+                width: int = 512, height: int = 512, scheduler: str = "DPMSolverMultistepScheduler",
+                text_embeddings: T.Optional[torch.Tensor] = None, uncond_embeddings: T.Optional[torch.Tensor] = None,
+                latents: T.Optional[torch.Tensor] = None, output_type: str = "pil") -> T.Dict[str, T.Any]:
+        """Text to image from pure noise: diffusers 0.9 `StableDiffusionPipeline.__call__` as the reference's text-to-audio
+        tasks run it (streamlit/util.py run_txt2img; SURVEY Appendix C).
+
+        `prompt`, `negative_prompt` and `seed` may be lists (a scalar is used for every clip): the clips run as one
+        batched CFG loop with per-clip text and unconditional embeddings and one generator per clip, so clip i equals a
+        single call with `seed[i]` up to the batch-size dependent accumulation order of the kernels.  Prompts are encoded
+        with the plain tokenizer + text encoder (`embed_text`, 77 tokens), the unconditional embedding is that of
+        `negative_prompt or ""`.  `text_embeddings` / `uncond_embeddings` / `latents` inject what would otherwise be
+        computed (B, 77, D) / (1 or B, 77, D) / (B, 4, height/8, width/8) fp16.  A fresh scheduler is built per call;
+        `self.scheduler`, which riffuse uses, is not touched.
+
+        Returns images (PIL list, or None for output_type="latent", or a float32 (B, H, W, 3) array for "np"),
+        latents (1/0.18215-scaled, what the VAE decodes), latents_unscaled and n_unet_evals."""
+        from riffusion.scheduler_b200 import get_scheduler
+
+        if height % 8 or width % 8:
+            raise ValueError(f"`height` and `width` have to be divisible by 8 but are {height} and {width}.")
+        if height % 64 or width % 64:
+            raise NotImplementedError(
+                f"height {height} / width {width}: sizes that are not multiples of 64 need up-sampling to odd sizes "
+                "(diffusers' upsample_size), which UNetB200 does not implement")
+        sched = get_scheduler(scheduler)
+        dev = self._device
+        as_list = lambda v: list(v) if isinstance(v, (list, tuple)) else None   # noqa: E731
+        lists = [v for v in (as_list(prompt), as_list(negative_prompt), as_list(seed)) if v is not None]
+        if text_embeddings is not None:
+            lists.append(list(range(text_embeddings.shape[0])))
+        if latents is not None:
+            lists.append(list(range(latents.shape[0])))
+        B = len(lists[0]) if lists else 1
+        if any(len(v) != B for v in lists):
+            raise ValueError("prompt, negative_prompt, seed, text_embeddings and latents must agree on the batch size")
+        per_clip = lambda v: as_list(v) if as_list(v) is not None else [v] * B   # noqa: E731
+
+        if text_embeddings is None:
+            if prompt is None:
+                raise ValueError("pass a prompt or text_embeddings")
+            text_embeddings = torch.cat([self.embed_text(p) for p in per_clip(prompt)])
+        text_embeddings = text_embeddings.to(device=dev, dtype=torch.float16)
+        do_cfg = guidance_scale > 1.0
+        if do_cfg:
+            if uncond_embeddings is None:
+                uncond_embeddings = torch.cat([self.embed_text(n or "") for n in per_clip(negative_prompt)])
+            uncond_embeddings = uncond_embeddings.to(device=dev, dtype=torch.float16)
+            uncond_embeddings = uncond_embeddings.expand(B, -1, -1) if uncond_embeddings.shape[0] == 1 else uncond_embeddings
+            context = torch.cat([uncond_embeddings, text_embeddings]).contiguous()
+        else:
+            context = text_embeddings.contiguous()
+
+        shape = (B, 4, height // 8, width // 8)
+        if latents is None:
+            latents = torch.cat([torch.randn((1,) + shape[1:], generator=torch.Generator(device=self.device).manual_seed(int(s)),
+                                             device=self.device, dtype=torch.float16) for s in per_clip(seed)])
+        latents = latents.to(device=dev, dtype=torch.float16).contiguous()
+        if tuple(latents.shape) != shape:
+            raise ValueError(f"latents must have shape {shape}, got {tuple(latents.shape)}")
+        # `latents * init_noise_sigma` is the identity: both schedulers have init_noise_sigma = 1
+
+        sched.set_timesteps(num_inference_steps)
+        graphed = self._graphed_unet(latents.shape, context) if self.use_cuda_graph and do_cfg else None
+        ctx_cache: T.Dict[str, T.Any] = {}
+        n_evals = 0
+        for t in sched.timesteps:
+            t_int = int(t)
+            if graphed is not None:
+                eps_pair = graphed(latents, t_int)
+            else:
+                model_in = torch.cat([latents] * 2) if do_cfg else latents
+                eps_pair = self.unet(model_in, t_int, encoder_hidden_states=context, ctx_cache=ctx_cache).sample
+            n_evals += 1
+            if not do_cfg:
+                eps_pair = torch.cat([eps_pair, eps_pair])
+            latents = sched.step_cfg(eps_pair, guidance_scale if do_cfg else 0.0, t_int, latents)
+
+        scaled = (1.0 / VAE_SCALE) * latents                                       # decode_latents: 1 / 0.18215 * latents
+        out: T.Dict[str, T.Any] = dict(latents=scaled, latents_unscaled=latents, n_unet_evals=n_evals, images=None)
+        if output_type == "latent" or self.vae is None:
+            return out
+        image = self.vae.decode(scaled).sample
+        if output_type == "pil":
+            # (image / 2 + 0.5).clamp(0, 1) in fp16, then .float(): numpy_to_pil's (x * 255).round() runs in fp32
+            u8 = ops.vae_image_to_u8(image, fp32_scale=True).cpu().numpy()
+            out["images"] = [Image.fromarray(im) for im in u8]
+        else:
+            out["images"] = (image / 2 + 0.5).clamp(0, 1).cpu().permute(0, 2, 3, 1).float().numpy()
+        return out
+
+    @torch.no_grad()
+    def text_to_audio_clips(self, prompt: T.Union[str, T.Sequence[str], None] = None, *, converter,
+                            init_angles: T.Optional[torch.Tensor] = None, height: T.Optional[int] = None,
+                            **txt2img_kwargs) -> T.Dict[str, torch.Tensor]:
+        """`txt2img` followed by the audio conversion without leaving the device: latents -> VAE decode -> uint8 image
+        (fp32 rounding, as txt2img's PIL images) -> mel amplitudes (mono = R plane) -> inverse mel + Griffin-Lim.  What
+        the reference's text-to-audio task does per clip (run_txt2img, then audio_segment_from_spectrogram_image) minus the
+        host round trip and `apply_filters`.  `converter` is a SpectrogramConverter; mono only, and `height` must be its
+        number of mel bins.  Returns device tensors: images (B, H, W, 3) uint8, waveform (B, 441 (W - 1)) fp32, latents,
+        latents_unscaled, n_unet_evals."""
+        p = converter.p
+        if p.stereo:
+            raise NotImplementedError("text_to_audio_clips is mono only; use txt2img + SpectrogramImageConverter for stereo")
+        height = p.num_frequencies if height is None else height
+        if height != p.num_frequencies:
+            raise ValueError(f"height {height} must equal the number of mel bins {p.num_frequencies}")
+        out = self.txt2img(prompt, height=height, output_type="latent", **txt2img_kwargs)
+        image = self.vae.decode(out["latents"]).sample
+        u8 = ops.vae_image_to_u8(image, fp32_scale=True)
+        return dict(images=u8, waveform=self._waveform_from_u8(u8, converter, init_angles), latents=out["latents"],
+                    latents_unscaled=out["latents_unscaled"], n_unet_evals=out["n_unet_evals"])
+
+    def _waveform_from_u8(self, u8: torch.Tensor, converter, init_angles: T.Optional[torch.Tensor]) -> torch.Tensor:
+        """(B, H, W, 3) uint8 spectrogram images on the device -> (B, hop (W - 1)) waveforms: image_util
+        spectrogram_from_image semantics (mono = R plane, max_value 30e6) + inverse mel + Griffin-Lim."""
+        from riffusion import _native
+
+        B, H, W, _ = u8.shape
+        mel = torch.empty((B, H, W), dtype=torch.float32, device=u8.device)
+        lib = _native.lib()
+        p = converter.p
+        for i in range(B):
+            _native.check(lib.rf_image_to_mel(u8[i].data_ptr(), H, W, 0, float(p.power_for_image), 30e6, mel[i].data_ptr(),
+                                              _native.stream_ptr(u8.device)))
+        return converter.waveform_from_mel_amplitudes(mel, init_angles)
+
     # ------------------------------------------------------------------------------ batched request -> audio
     @torch.no_grad()
     def generate_clips(self, text_embeddings: torch.Tensor, uncond_embeddings: torch.Tensor, init_latents: torch.Tensor,
@@ -323,8 +456,6 @@ class RiffusionPipeline:
         This is what `server.compute_request` does per request (riffuse, then audio_from_spectrogram_image,
         server.py:145-164) without leaving the GPU in between.  Returns device tensors:
         images (B,512,512,3) uint8, waveform (B, L) fp32, latents."""
-        from riffusion import _native
-
         out = self.interpolate_img2img(
             text_embeddings=text_embeddings, init_latents=init_latents, generator_a=None, generator_b=None,
             interpolate_alpha=0.0, strength_a=strength, strength_b=strength, num_inference_steps=num_inference_steps,
@@ -332,14 +463,7 @@ class RiffusionPipeline:
         latents = out["latents_unscaled"]
         image = self.vae.decode(out["latents"]).sample
         u8 = ops.vae_image_to_u8(image)
-        B, H, W, _ = u8.shape
-        mel = torch.empty((B, H, W), dtype=torch.float32, device=u8.device)
-        lib = _native.lib()
-        p = converter.p
-        for i in range(B):
-            _native.check(lib.rf_image_to_mel(u8[i].data_ptr(), H, W, 0, float(p.power_for_image), 30e6, mel[i].data_ptr(),
-                                              _native.stream_ptr(u8.device)))
-        wave = converter.waveform_from_mel_amplitudes(mel, init_angles)
+        wave = self._waveform_from_u8(u8, converter, init_angles)
         return dict(images=u8, waveform=wave, latents=out["latents"], latents_unscaled=latents,
                     n_unet_evals=out["n_unet_evals"])
 

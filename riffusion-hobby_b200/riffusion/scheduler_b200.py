@@ -1,4 +1,4 @@
-"""PNDM (PLMS) scheduler for the denoising loop — host-side tables + one fused device step.
+"""PNDM (PLMS) and DPM-Solver++ schedulers for the denoising loop — host-side tables + one fused device step.
 
 Restates diffusers 0.9 `PNDMScheduler(skip_prk_steps=True, steps_offset=1, beta_schedule="scaled_linear",
 beta_start=0.00085, beta_end=0.012, set_alpha_to_one=False)` [memory; SURVEY Appendix B], i.e. the scheduler
@@ -100,3 +100,98 @@ class PNDMSchedulerB200:
         """diffusers-compatible signature: the model output is already guided."""
         pair = torch.cat([model_output, model_output]).contiguous()     # eps_u == eps_t  =>  guided eps == eps
         return types.SimpleNamespace(prev_sample=self.step_cfg(pair, 0.0, int(timestep), sample))
+
+
+class DPMSolverMultistepSchedulerB200:
+    """DPM-Solver++(2M): diffusers 0.9 `DPMSolverMultistepScheduler.from_config(<the PNDM config above>)`, i.e.
+    algorithm_type="dpmsolver++", solver_type="midpoint", solver_order=2, lower_order_final=True, epsilon prediction, no
+    thresholding [memory; SURVEY Appendix C].  The reference's default txt2img scheduler (streamlit/util.py:26-33).
+
+    The tables and per-step scalars are computed on the host with fp32 torch ops, as the reference computes them; the
+    tensor update runs in one kernel fused with the guidance combine (`rf_cfg_dpmpp_step_f16`).  The x0 history lives
+    in two ping-pong buffers: step i reads the buffer step i-1 wrote and writes the other one."""
+    order = 1
+
+    def __init__(self, num_train_timesteps: int = 1000, beta_start: float = 0.00085, beta_end: float = 0.012):
+        betas = torch.linspace(beta_start ** 0.5, beta_end ** 0.5, num_train_timesteps, dtype=torch.float32) ** 2
+        self.alphas_cumprod = torch.cumprod(1.0 - betas, dim=0)
+        self.alpha_t = torch.sqrt(self.alphas_cumprod)
+        self.sigma_t = torch.sqrt(1 - self.alphas_cumprod)
+        self.lambda_t = torch.log(self.alpha_t) - torch.log(self.sigma_t)
+        self.num_train_timesteps = num_train_timesteps
+        self.config = {"num_train_timesteps": num_train_timesteps, "solver_order": 2, "lower_order_final": True}
+        self.init_noise_sigma = 1.0
+        self.timesteps: T.Optional[torch.Tensor] = None
+        self.set_timesteps(50)
+
+    def set_timesteps(self, num_inference_steps: int, device=None) -> None:
+        """`linspace(0, 999, n + 1).round()[::-1][:-1]`: n timesteps from 999 down, `steps_offset` is not used."""
+        self.num_inference_steps = num_inference_steps
+        ts = np.linspace(0, self.num_train_timesteps - 1, num_inference_steps + 1).round()[::-1][:-1].copy()
+        self.timesteps = torch.from_numpy(ts.astype(np.int64))
+        self.lower_order_nums = 0
+        self._x0_bufs: T.Optional[T.List[torch.Tensor]] = None
+        self._x0_prev: T.Optional[torch.Tensor] = None
+        self._slot = 0
+
+    def scale_model_input(self, sample: torch.Tensor, timestep=None) -> torch.Tensor:
+        return sample
+
+    def coefficients(self, timestep: int) -> T.Dict[str, T.Any]:
+        """Scalars of the step at `timestep`, each a 0-dim fp32 torch result as in the reference, returned as floats."""
+        ts = self.timesteps.tolist()
+        i = ts.index(int(timestep))
+        t = ts[i + 1] if i + 1 < len(ts) else 0
+        s0 = ts[i]
+        lower_order_final = i == len(ts) - 1 and self.config["lower_order_final"] and len(ts) < 15
+        second = not (self.lower_order_nums < 1 or lower_order_final)
+        h = self.lambda_t[t] - self.lambda_t[s0]
+        c_0 = self.alpha_t[t] * (torch.exp(-h) - 1.0)
+        co = dict(second=second, sigma_s=float(self.sigma_t[s0]), alpha_s=float(self.alpha_t[s0]),
+                  c_x=float(self.sigma_t[t] / self.sigma_t[s0]), c_0=float(c_0), inv_r0=0.0, c_d1=0.0)
+        if second:
+            h_0 = self.lambda_t[s0] - self.lambda_t[ts[i - 1]]
+            r0 = h_0 / h
+            co.update(inv_r0=float(1.0 / r0), c_d1=float(0.5 * c_0))
+        return co
+
+    def step_cfg(self, eps_pair: torch.Tensor, guidance: float, timestep: int, sample: torch.Tensor) -> torch.Tensor:
+        """Guidance combine + scheduler.step in one kernel.  eps_pair = UNet output for [uncond | text]."""
+        co = self.coefficients(timestep)
+        sample = sample.contiguous()
+        if self._x0_bufs is None or self._x0_bufs[0].shape != sample.shape or self._x0_bufs[0].device != sample.device:
+            self._x0_bufs = [torch.empty_like(sample), torch.empty_like(sample)]
+        x0_out = self._x0_bufs[self._slot]
+        _, prev = ops.cfg_dpmpp_step(eps_pair.contiguous(), guidance, sample, self._x0_prev if co["second"] else None,
+                                     co["sigma_s"], co["alpha_s"], co["c_x"], co["c_0"], co["inv_r0"], co["c_d1"],
+                                     x0_out=x0_out)
+        self._x0_prev, self._slot = x0_out, self._slot ^ 1
+        self.lower_order_nums = min(self.lower_order_nums + 1, self.config["solver_order"])
+        return prev
+
+    def step(self, model_output: torch.Tensor, timestep, sample: torch.Tensor, **kwargs):
+        """diffusers-compatible signature: the model output is already guided."""
+        pair = torch.cat([model_output, model_output]).contiguous()     # eps_u == eps_t  =>  guided eps == eps
+        return types.SimpleNamespace(prev_sample=self.step_cfg(pair, 0.0, int(timestep), sample))
+
+
+# the reference's scheduler menu (streamlit/util.py:26-33); index 0 is its default
+SCHEDULER_OPTIONS = [
+    "DPMSolverMultistepScheduler",
+    "PNDMScheduler",
+    "DDIMScheduler",
+    "LMSDiscreteScheduler",
+    "EulerDiscreteScheduler",
+    "EulerAncestralDiscreteScheduler",
+]
+
+
+def get_scheduler(name: str):
+    """A fresh scheduler for `name` (streamlit/util.py:80-109), configured from SD-1.5's PNDM config."""
+    if name == "DPMSolverMultistepScheduler":
+        return DPMSolverMultistepSchedulerB200()
+    if name == "PNDMScheduler":
+        return PNDMSchedulerB200()
+    if name in SCHEDULER_OPTIONS:
+        raise NotImplementedError(f"{name} has no B200 implementation; use DPMSolverMultistepScheduler or PNDMScheduler")
+    raise ValueError(f"Unknown scheduler {name}")

@@ -308,6 +308,28 @@ def cfg_pndm_step(eps_pair, guidance, hist, coef, sample, ca, cb, want_eps=True)
     return eps_out, prev
 
 
+def cfg_dpmpp_step(eps_pair, guidance, sample, x0_prev, sigma_s, alpha_s, c_x, c_0, inv_r0=0.0, c_d1=0.0, x0_out=None,
+                   out=None):
+    """Guidance combine + one DPM-Solver++ update (rf_cfg_dpmpp_step_f16).  eps_pair: (2B, ...) fp16 [uncond | text];
+    x0_prev: the previous step's x0 prediction (second order) or None (first order).  Returns (x0 prediction, prev_sample);
+    `x0_out` / `out` receive them when given (`out` may be `sample`)."""
+    _f16(eps_pair, "eps_pair"), _f16(sample, "sample")
+    n = sample.numel()
+    assert eps_pair.numel() == 2 * n and eps_pair.is_contiguous() and sample.is_contiguous()
+    for t in (x0_prev, x0_out, out):
+        if t is not None:
+            _f16(t, "history / output")
+            assert t.numel() == n and t.is_contiguous()
+    x0_out = torch.empty_like(sample) if x0_out is None else x0_out
+    out = torch.empty_like(sample) if out is None else out
+    with torch.cuda.device(sample.device):
+        _native.check(_native.lib().rf_cfg_dpmpp_step_f16(
+            eps_pair.data_ptr(), n, float(guidance), sample.data_ptr(), None if x0_prev is None else x0_prev.data_ptr(),
+            float(sigma_s), float(alpha_s), float(c_x), float(c_0), float(inv_r0), float(c_d1), x0_out.data_ptr(),
+            out.data_ptr(), _stream(sample)))
+    return x0_out, out
+
+
 def axpby(x, noise, a, b, mask=None, z=None):
     _f16(x, "x")
     y = torch.empty_like(x)
@@ -344,14 +366,16 @@ def attention(q: torch.Tensor, k: torch.Tensor, vt: torch.Tensor, heads: int, nk
     return out
 
 
-def vae_image_to_u8(x_nchw: torch.Tensor) -> torch.Tensor:
-    """(B, 3, H, W) fp16 in [-1, 1] -> (B, H, W, 3) uint8, the array PIL images are built from."""
+def vae_image_to_u8(x_nchw: torch.Tensor, fp32_scale: bool = False) -> torch.Tensor:
+    """(B, 3, H, W) fp16 in [-1, 1] -> (B, H, W, 3) uint8, the array PIL images are built from.  `fp32_scale`: `* 255`
+    and the round in fp32, as the txt2img pipeline does; otherwise in fp16, as the img2img pipeline does."""
     _f16(x_nchw, "x")
     B, Cc, H, W = x_nchw.shape
     assert Cc == 3
     y = torch.empty((B, H, W, 3), dtype=torch.uint8, device=x_nchw.device)
+    fn = _native.lib().rf_vae_image_to_u8_f32scale if fp32_scale else _native.lib().rf_vae_image_to_u8
     with torch.cuda.device(x_nchw.device):
-        _native.check(_native.lib().rf_vae_image_to_u8(x_nchw.contiguous().data_ptr(), B, H, W, y.data_ptr(), _stream(x_nchw)))
+        _native.check(fn(x_nchw.contiguous().data_ptr(), B, H, W, y.data_ptr(), _stream(x_nchw)))
     return y
 
 
