@@ -306,6 +306,23 @@ int rf_cfg_dpmpp_step_f16(const void* eps_pair, long n, float guidance, const vo
 int rf_axpby_f16(const void* x, const void* noise, float a, float b, const void* mask, const void* z, long n,
                  void* y, void* stream);
 
+/* diffusers 0.9 add_noise with its fp16 op sequence: y = s * x + s1 * noise, rounded to fp16 after each op.  s and s1 are
+ * the fp16 values alphas_cumprod[t] ** 0.5 and (1 - alphas_cumprod[t]) ** 0.5 with alphas_cumprod cast to fp16 first
+ * (img2img's prepare_latents); values not representable in fp16 are rejected.  x, noise, y: n fp16; y may alias x. */
+int rf_add_noise_f16_seq(const void* x, const void* noise, float s, float s1, long n, void* y, void* stream);
+
+/* ---- spectrogram-image glue of audio to audio (rf_image_ops.cu) ---- */
+/* Pillow-exact Image.resize(..., BICUBIC) of B uint8 RGB images: x (B, H_in, W_in, 3) -> y (B, H_out, W_out, 3), NHWC.
+ * Horizontal pass, then vertical, each skipped when its size is unchanged; taps in int32 fixed point with 22 fractional
+ * bits, built on the host as Pillow builds them and cached on the device per (device, n_in, n_out).  y must not alias x. */
+int rf_resample_u8(const uint8_t* x_nhwc, int B, int H_in, int W_in, int H_out, int W_out, uint8_t* y_nhwc, void* stream);
+/* Host only: the fixed-point taps rf_resample_u8 uses along one axis of n_in -> n_out pixels.  *ksize receives the taps
+ * per output pixel; bounds (optional, [n_out][2] = first input pixel, tap count) and kk (optional, [n_out][ksize]) are
+ * filled when given. */
+int rf_resample_coeffs(int n_in, int n_out, int* ksize, int32_t* bounds, int32_t* kk);
+/* img2img preprocess: uint8 NHWC (B, H, W, 3) -> fp16 NCHW (B, 3, H, W), 2 * (u / 255) - 1 in fp32 rounded once to fp16 */
+int rf_image_u8_to_f16(const uint8_t* x_nhwc, int B, int H, int W, void* y_nchw, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

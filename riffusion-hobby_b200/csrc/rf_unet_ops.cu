@@ -7,6 +7,7 @@
 // 0.9 [restated from memory, package absent]): torch.nn.GroupNorm / LayerNorm / F.gelu / softmax /
 // F.interpolate(nearest) / Conv2d, PNDMScheduler.step, classifier-free guidance combine.
 #include <cuda_fp16.h>
+#include <cmath>
 #include <cstdlib>
 #include <cuda_runtime.h>
 
@@ -666,6 +667,31 @@ __global__ void k_axpby(const __half* __restrict__ x, const __half* __restrict__
     }
 }
 
+// diffusers 0.9 `add_noise` on fp16 tensors (DDPM / PNDM / DPM-Solver share it): alphas_cumprod is cast to the sample
+// dtype, s = a[t] ** 0.5 and s1 = (1 - a[t]) ** 0.5 are fp16 values (computed on the host), and
+//   y = s * x + s1 * n
+// rounds to fp16 after every op (each op widens to fp32 and rounds its result once, as torch does).  n8 elements (a
+// multiple of 8, every stream 16-byte aligned) in 16-byte groups, the remaining n - n8 < 8 one by one.
+__device__ __forceinline__ __half add_noise_elem(__half x, __half nz, float s, float s1) {
+    return rn(wf(rn(s * wf(x))) + wf(rn(s1 * wf(nz))));
+}
+
+__global__ void k_add_noise_seq(const __half* x, const __half* nz, float s, float s1, size_t n, size_t n8, __half* y) {
+    const size_t tid = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    const size_t stride = static_cast<size_t>(gridDim.x) * blockDim.x;
+    for (size_t gi = tid; gi < n8 / 8; gi += stride) {
+        const size_t i = gi * 8;
+        union V8 { uint4 u; __half h[8]; };
+        V8 a, b, o;
+        a.u = *reinterpret_cast<const uint4*>(x + i);
+        b.u = *reinterpret_cast<const uint4*>(nz + i);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) o.h[k] = add_noise_elem(a.h[k], b.h[k], s, s1);
+        *reinterpret_cast<uint4*>(y + i) = o.u;
+    }
+    for (size_t i = n8 + tid; i < n; i += stride) y[i] = add_noise_elem(x[i], nz[i], s, s1);
+}
+
 // channel concatenation of two NHWC tensors (torch.cat([a, b], dim=1) in NCHW terms)
 __global__ void k_concat_channels(const __half* __restrict__ a, const __half* __restrict__ b, size_t pixels, int Ca,
                                   int Cb, __half* __restrict__ y) {
@@ -1074,5 +1100,19 @@ extern "C" int rf_axpby_f16(const void* x, const void* noise, float a, float b, 
         static_cast<const __half*>(x), static_cast<const __half*>(noise), a, b, static_cast<const __half*>(mask),
         static_cast<const __half*>(z), static_cast<size_t>(n), static_cast<__half*>(y));
     RF_CUDA_LAUNCH_CHECK("k_axpby");
+    return RF_OK;
+}
+
+extern "C" int rf_add_noise_f16_seq(const void* x, const void* noise, float s, float s1, long n, void* y, void* stream) {
+    // s and s1 are the fp16 values a[t] ** 0.5 and (1 - a[t]) ** 0.5: anything not representable in fp16 is a caller bug
+    const auto is_f16 = [](float v) { return std::isfinite(v) && __half2float(__float2half_rn(v)) == v; };
+    if (!x || !noise || !y || n <= 0 || !is_f16(s) || !is_f16(s1))
+        return rf_fail(RF_ERR_INVALID, "rf_add_noise_f16_seq: bad argument");
+    const size_t N = static_cast<size_t>(n);
+    const auto a16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+    const size_t n8 = (a16(x) && a16(noise) && a16(y)) ? (N & ~static_cast<size_t>(7)) : 0;
+    k_add_noise_seq<<<grid_for(n8 / 8 + (N - n8), 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+        static_cast<const __half*>(x), static_cast<const __half*>(noise), s, s1, N, n8, static_cast<__half*>(y));
+    RF_CUDA_LAUNCH_CHECK("k_add_noise_seq");
     return RF_OK;
 }

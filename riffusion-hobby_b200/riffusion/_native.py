@@ -127,6 +127,10 @@ SIGNATURES = {
                                         C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rf_axpby_f16":(C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_long,
                                C.c_void_p, C.c_void_p]),
+    "rf_add_noise_f16_seq": (C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_long, C.c_void_p, C.c_void_p]),
+    "rf_resample_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "rf_resample_coeffs": (C.c_int, [C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rf_image_u8_to_f16": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "rf_attention_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.c_int, C.c_int, C.c_float, C.c_void_p]),
     "rf_attention_masked_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,

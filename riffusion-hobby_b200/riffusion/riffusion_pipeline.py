@@ -267,23 +267,13 @@ class RiffusionPipeline:
         del accepts_eta
         t_start = max(num_inference_steps - init_timestep + offset, 0)                             # :392
         timesteps = self.scheduler.timesteps[t_start:]
-        ctx_cache: T.Dict[str, T.Any] = {}
-        graphed = self._graphed_unet(latents.shape, context) if self.use_cuda_graph and do_cfg else None
-        n_evals = 0
-        for t in timesteps:                                                                        # :398
-            t_int = int(t)
-            if graphed is not None:
-                eps_pair = graphed(latents, t_int)
-            else:
-                model_in = torch.cat([latents] * 2) if do_cfg else latents                         # :400-403
-                eps_pair = self.unet(model_in, t_int, encoder_hidden_states=context, ctx_cache=ctx_cache).sample
-            n_evals += 1
-            if not do_cfg:
-                eps_pair = torch.cat([eps_pair, eps_pair])
-            latents = self.scheduler.step_cfg(eps_pair, guidance_scale if do_cfg else 0.0, t_int, latents)   # :411-418
-            if mask is not None:                                                                   # :420-425
-                m = mask.to(device=dev, dtype=latents_dtype).expand_as(latents).contiguous()
-                latents = self.scheduler.add_noise(init_latents_orig, noise, t_int, mask=m, blend_with=latents)
+        mask_blend = None
+        if mask is not None:                                                                       # :420-425
+            def mask_blend(x: torch.Tensor, t_int: int) -> torch.Tensor:
+                m = mask.to(device=dev, dtype=latents_dtype).expand_as(x).contiguous()
+                return self.scheduler.add_noise(init_latents_orig, noise, t_int, mask=m, blend_with=x)
+        latents, n_evals = self._denoise(self.scheduler, latents, context, timesteps, guidance_scale,  # :398-418
+                                         mask_blend)
 
         # :427 — the reference rescales in fp16 (`1.0 / 0.18215 * latents`) and returns THAT tensor under "latents"; the
         # un-scaled loop state and the evaluation count are extra keys of this implementation
@@ -314,6 +304,32 @@ class RiffusionPipeline:
         else:
             graphed.set_context(context)
         return graphed
+
+    def _denoise(self, sched, latents: torch.Tensor, context: torch.Tensor, timesteps, guidance_scale: float,
+                 after_step: T.Optional[T.Callable[[torch.Tensor, int], torch.Tensor]] = None
+                 ) -> T.Tuple[torch.Tensor, int]:
+        """The denoising loop of interpolate_img2img, txt2img and img2img: one CFG UNet evaluation per timestep (a CUDA
+        graph replay when enabled, [uncond | text] doubled batch; text only when guidance <= 1), then the fused guidance +
+        scheduler step.  `after_step(latents, t)` runs after each step (riffuse's mask blend).  Returns (latents,
+        number of UNet evaluations)."""
+        do_cfg = guidance_scale > 1.0
+        graphed = self._graphed_unet(latents.shape, context) if self.use_cuda_graph and do_cfg else None
+        ctx_cache: T.Dict[str, T.Any] = {}
+        n_evals = 0
+        for t in timesteps:
+            t_int = int(t)
+            if graphed is not None:
+                eps_pair = graphed(latents, t_int)
+            else:
+                model_in = torch.cat([latents] * 2) if do_cfg else latents
+                eps_pair = self.unet(model_in, t_int, encoder_hidden_states=context, ctx_cache=ctx_cache).sample
+            n_evals += 1
+            if not do_cfg:
+                eps_pair = torch.cat([eps_pair, eps_pair])
+            latents = sched.step_cfg(eps_pair, guidance_scale if do_cfg else 0.0, t_int, latents)
+            if after_step is not None:
+                latents = after_step(latents, t_int)
+        return latents, n_evals
 
     # ------------------------------------------------------------------------------ txt2img
     @torch.no_grad()
@@ -346,31 +362,8 @@ class RiffusionPipeline:
                 "(diffusers' upsample_size), which UNetB200 does not implement")
         sched = get_scheduler(scheduler)
         dev = self._device
-        as_list = lambda v: list(v) if isinstance(v, (list, tuple)) else None   # noqa: E731
-        lists = [v for v in (as_list(prompt), as_list(negative_prompt), as_list(seed)) if v is not None]
-        if text_embeddings is not None:
-            lists.append(list(range(text_embeddings.shape[0])))
-        if latents is not None:
-            lists.append(list(range(latents.shape[0])))
-        B = len(lists[0]) if lists else 1
-        if any(len(v) != B for v in lists):
-            raise ValueError("prompt, negative_prompt, seed, text_embeddings and latents must agree on the batch size")
-        per_clip = lambda v: as_list(v) if as_list(v) is not None else [v] * B   # noqa: E731
-
-        if text_embeddings is None:
-            if prompt is None:
-                raise ValueError("pass a prompt or text_embeddings")
-            text_embeddings = torch.cat([self.embed_text(p) for p in per_clip(prompt)])
-        text_embeddings = text_embeddings.to(device=dev, dtype=torch.float16)
-        do_cfg = guidance_scale > 1.0
-        if do_cfg:
-            if uncond_embeddings is None:
-                uncond_embeddings = torch.cat([self.embed_text(n or "") for n in per_clip(negative_prompt)])
-            uncond_embeddings = uncond_embeddings.to(device=dev, dtype=torch.float16)
-            uncond_embeddings = uncond_embeddings.expand(B, -1, -1) if uncond_embeddings.shape[0] == 1 else uncond_embeddings
-            context = torch.cat([uncond_embeddings, text_embeddings]).contiguous()
-        else:
-            context = text_embeddings.contiguous()
+        B, per_clip, context = self._batch_context(prompt, negative_prompt, seed, text_embeddings, uncond_embeddings,
+                                                   guidance_scale, latents=None if latents is None else latents.shape[0])
 
         shape = (B, 4, height // 8, width // 8)
         if latents is None:
@@ -382,33 +375,170 @@ class RiffusionPipeline:
         # `latents * init_noise_sigma` is the identity: both schedulers have init_noise_sigma = 1
 
         sched.set_timesteps(num_inference_steps)
-        graphed = self._graphed_unet(latents.shape, context) if self.use_cuda_graph and do_cfg else None
-        ctx_cache: T.Dict[str, T.Any] = {}
-        n_evals = 0
-        for t in sched.timesteps:
-            t_int = int(t)
-            if graphed is not None:
-                eps_pair = graphed(latents, t_int)
-            else:
-                model_in = torch.cat([latents] * 2) if do_cfg else latents
-                eps_pair = self.unet(model_in, t_int, encoder_hidden_states=context, ctx_cache=ctx_cache).sample
-            n_evals += 1
-            if not do_cfg:
-                eps_pair = torch.cat([eps_pair, eps_pair])
-            latents = sched.step_cfg(eps_pair, guidance_scale if do_cfg else 0.0, t_int, latents)
+        latents, n_evals = self._denoise(sched, latents, context, sched.timesteps, guidance_scale)
+        return self._decode_output(latents, n_evals, output_type)
 
-        scaled = (1.0 / VAE_SCALE) * latents                                       # decode_latents: 1 / 0.18215 * latents
+    def _batch_context(self, prompt, negative_prompt, seed, text_embeddings, uncond_embeddings, guidance_scale: float,
+                       **batch_sizes: T.Optional[int]):
+        """Batch size, per-clip broadcast and CFG context of txt2img / img2img.  `prompt`, `negative_prompt` and `seed`
+        may be lists; the batch size is their common length, which the first dimension of `text_embeddings` and the
+        `batch_sizes` given (None entries are ignored) must equal.  Returns (B, per_clip, context) with context = [uncond | text]
+        (text only when guidance <= 1)."""
+        dev = self._device
+        as_list = lambda v: list(v) if isinstance(v, (list, tuple)) else None   # noqa: E731
+        lists = [v for v in (as_list(prompt), as_list(negative_prompt), as_list(seed)) if v is not None]
+        if text_embeddings is not None:
+            lists.append(list(range(text_embeddings.shape[0])))
+        for n in batch_sizes.values():
+            if n is not None:
+                lists.append(list(range(n)))
+        B = len(lists[0]) if lists else 1
+        if any(len(v) != B for v in lists):
+            raise ValueError(f"prompt, negative_prompt, seed, text_embeddings and {', '.join(batch_sizes)} must agree on the "
+                             "batch size")
+        per_clip = lambda v: as_list(v) if as_list(v) is not None else [v] * B   # noqa: E731
+
+        if text_embeddings is None:
+            if prompt is None:
+                raise ValueError("pass a prompt or text_embeddings")
+            text_embeddings = torch.cat([self.embed_text(p) for p in per_clip(prompt)])
+        text_embeddings = text_embeddings.to(device=dev, dtype=torch.float16)
+        if guidance_scale > 1.0:
+            if uncond_embeddings is None:
+                uncond_embeddings = torch.cat([self.embed_text(n or "") for n in per_clip(negative_prompt)])
+            uncond_embeddings = uncond_embeddings.to(device=dev, dtype=torch.float16)
+            uncond_embeddings = uncond_embeddings.expand(B, -1, -1) if uncond_embeddings.shape[0] == 1 else uncond_embeddings
+            context = torch.cat([uncond_embeddings, text_embeddings]).contiguous()
+        else:
+            context = text_embeddings.contiguous()
+        return B, per_clip, context
+
+    def _decode_output(self, latents: torch.Tensor, n_evals: int, output_type: str) -> T.Dict[str, T.Any]:
+        """decode_latents of txt2img / img2img: 1 / 0.18215 * latents, VAE decode, (image / 2 + 0.5).clamp(0, 1) in fp16,
+        then `.float()`, so numpy_to_pil's (x * 255).round() runs in fp32."""
+        scaled = (1.0 / VAE_SCALE) * latents
         out: T.Dict[str, T.Any] = dict(latents=scaled, latents_unscaled=latents, n_unet_evals=n_evals, images=None)
         if output_type == "latent" or self.vae is None:
             return out
         image = self.vae.decode(scaled).sample
         if output_type == "pil":
-            # (image / 2 + 0.5).clamp(0, 1) in fp16, then .float(): numpy_to_pil's (x * 255).round() runs in fp32
             u8 = ops.vae_image_to_u8(image, fp32_scale=True).cpu().numpy()
             out["images"] = [Image.fromarray(im) for im in u8]
         else:
             out["images"] = (image / 2 + 0.5).clamp(0, 1).cpu().permute(0, 2, 3, 1).float().numpy()
         return out
+
+    # ------------------------------------------------------------------------------ img2img
+    @torch.no_grad()
+    def img2img(self, prompt: T.Union[str, T.Sequence[str], None] = None, *,
+                init_image: T.Union[Image.Image, T.Sequence[Image.Image], None] = None,
+                init_images_u8: T.Optional[torch.Tensor] = None, strength: float = 0.8, num_inference_steps: int = 50,
+                guidance_scale: float = 7.5, negative_prompt: T.Union[str, T.Sequence[T.Optional[str]], None] = None,
+                seed: T.Union[int, T.Sequence[int]] = 42, scheduler: str = "DPMSolverMultistepScheduler",
+                text_embeddings: T.Optional[torch.Tensor] = None, uncond_embeddings: T.Optional[torch.Tensor] = None,
+                noise: T.Optional[torch.Tensor] = None, output_type: str = "pil") -> T.Dict[str, T.Any]:
+        """Image to image: diffusers 0.9 `StableDiffusionImg2ImgPipeline.__call__` as the reference's audio-to-audio task
+        runs it (streamlit/util.py run_img2img; SURVEY Appendix D).
+
+        The init image is a PIL image (or one per clip), preprocessed on the host as `preprocess_image` does, or
+        `init_images_u8`, a (1 or B, H, W, 3) uint8 tensor whose sides are multiples of 32, converted on the device with
+        the same arithmetic.  Each clip draws from one generator seeded with its seed: the VAE posterior sample first,
+        then the noise.  The noise is added at timesteps[t_start] with the fp16 op sequence of `add_noise`, and the loop
+        runs timesteps[t_start:] with a fresh scheduler (`self.scheduler`, which riffuse uses, is not touched).
+        `prompt`, `negative_prompt` and `seed` may be lists, batched as in `txt2img`; `text_embeddings`,
+        `uncond_embeddings` and `noise` ((B, 4, H/8, W/8) fp16, replacing the second draw) inject what would otherwise
+        be computed.
+
+        Returns images (PIL list, None for output_type="latent", or a float32 (B, H, W, 3) array for "np"), latents
+        (1/0.18215-scaled), latents_unscaled and n_unet_evals."""
+        from riffusion.scheduler_b200 import get_scheduler
+        from riffusion.vae_b200 import _Posterior
+
+        if (init_image is None) == (init_images_u8 is None):
+            raise ValueError("pass exactly one of init_image and init_images_u8")
+        dev = self._device
+        if init_images_u8 is not None:
+            if init_images_u8.dim() != 4 or init_images_u8.shape[-1] != 3 or init_images_u8.dtype != torch.uint8:
+                raise ValueError(f"init_images_u8 must be a (B, H, W, 3) uint8 tensor, got {tuple(init_images_u8.shape)} "
+                                 f"{init_images_u8.dtype}")
+            if init_images_u8.shape[1] % 32 or init_images_u8.shape[2] % 32:
+                raise ValueError(f"init_images_u8 sides must be multiples of 32, got {tuple(init_images_u8.shape[1:3])}")
+            height, width = int(init_images_u8.shape[1]), int(init_images_u8.shape[2])
+        else:
+            imgs = [init_image] if isinstance(init_image, Image.Image) else list(init_image)
+            width, height = (x - x % 32 for x in imgs[0].size)
+        if height % 64 or width % 64:
+            raise NotImplementedError(
+                f"height {height} / width {width}: sizes that are not multiples of 64 need up-sampling to odd sizes "
+                "(diffusers' upsample_size), which UNetB200 does not implement")
+        sched = get_scheduler(scheduler)
+        _, timesteps, t_noise = sched.img2img_timesteps(num_inference_steps, strength)
+        n_img = init_images_u8.shape[0] if init_images_u8 is not None else len(imgs)
+        B, per_clip, context = self._batch_context(prompt, negative_prompt, seed, text_embeddings, uncond_embeddings,
+                                                   guidance_scale, noise=None if noise is None else noise.shape[0],
+                                                   init_images=None if n_img == 1 else n_img)
+
+        if init_images_u8 is not None:
+            image = ops.image_u8_to_f16(init_images_u8.to(dev))
+        else:
+            image = torch.cat([preprocess_image(im) for im in imgs]).to(device=dev, dtype=torch.float16)
+        mean, logvar = self.vae.encode_moments(image)                       # one batched encoder pass
+        lats, noises = [], []
+        for i, s in enumerate(per_clip(seed)):
+            g = torch.Generator(device=self.device).manual_seed(int(s))
+            j = i if n_img > 1 else 0
+            lats.append(VAE_SCALE * _Posterior(mean[j:j + 1], logvar[j:j + 1]).sample(generator=g))
+            if noise is None:
+                noises.append(torch.randn(lats[-1].shape, generator=g, device=self.device, dtype=torch.float16))
+        init_latents = torch.cat(lats).contiguous()
+        noise = torch.cat(noises) if noise is None else noise.to(device=dev, dtype=torch.float16).contiguous()
+        if noise.shape != init_latents.shape:
+            raise ValueError(f"noise must have shape {tuple(init_latents.shape)}, got {tuple(noise.shape)}")
+        latents = sched.add_noise_fp16(init_latents, noise, t_noise)
+        latents, n_evals = self._denoise(sched, latents, context, timesteps, guidance_scale)
+        return self._decode_output(latents, n_evals, output_type)
+
+    @torch.no_grad()
+    def audio_to_audio_clips(self, waveforms: torch.Tensor, *, converter, prompt: T.Union[str, T.Sequence[str], None] = None,
+                             init_angles: T.Optional[torch.Tensor] = None, **img2img_kwargs) -> T.Dict[str, T.Any]:
+        """img2img on a batch of equally long mono clips without leaving the device, what the reference's audio-to-audio
+        task does one clip at a time: waveform -> mel amplitudes (rf_stft_mel) -> spectrogram image (rf_mel_to_image) ->
+        Pillow-exact BICUBIC resize to the next multiples of 32 (rf_resample_u8) -> `img2img` -> uint8 image (fp32
+        rounding) -> BICUBIC resize back -> mel amplitudes (mono = R plane, max_value 30e6) -> inverse mel + Griffin-Lim.
+
+        `waveforms`: (B, L) float32 samples at the converter's rate, int16-valued as `spectrogram_from_audio` reads them.
+        `converter` is a mono SpectrogramConverter.  The img2img keywords (strength, seed, num_inference_steps, ...) pass
+        through.  Returns device tensors: source_images and images (B, H, W, 3) uint8, waveform (B, hop (W - 1)) fp32,
+        latents, latents_unscaled, and n_unet_evals."""
+        from riffusion import _native
+
+        p = converter.p
+        if p.stereo:
+            raise NotImplementedError("audio_to_audio_clips is mono only (no 20 kHz stereo on the device path); use "
+                                      "img2img with SpectrogramImageConverter images for stereo")
+        L = int(waveforms.shape[-1])
+        H, W = p.num_frequencies, 1 + L // p.hop_length
+        H32, W32 = (-(-v // 32) * 32 for v in (H, W))
+        if H32 % 64 or W32 % 64:
+            raise NotImplementedError(
+                f"clips of {L} samples give {H} x {W} images, {H32} x {W32} after the 32-stride resize: sizes that are "
+                "not multiples of 64 need up-sampling to odd sizes (diffusers' upsample_size), which UNetB200 does not "
+                "implement")
+        wave = _native.require_cuda(waveforms, "waveforms", torch.float32)
+        wave = wave[None] if wave.dim() == 1 else wave
+        B = wave.shape[0]
+        mel = converter.mel_amplitudes_from_waveform(wave)
+        src = torch.empty((B, H, W, 3), dtype=torch.uint8, device=wave.device)
+        mx = torch.empty((B,), dtype=torch.float32, device=wave.device)
+        lib = _native.lib()
+        for i in range(B):
+            _native.check(lib.rf_mel_to_image(mel[i].data_ptr(), 1, H, W, float(p.power_for_image), src[i].data_ptr(),
+                                              mx[i:i + 1].data_ptr(), _native.stream_ptr(wave.device)))
+        out = self.img2img(prompt, init_images_u8=ops.resample_u8(src, H32, W32), output_type="latent",
+                           **img2img_kwargs)
+        riffed = ops.resample_u8(ops.vae_image_to_u8(self.vae.decode(out["latents"]).sample, fp32_scale=True), H, W)
+        return dict(source_images=src, images=riffed, waveform=self._waveform_from_u8(riffed, converter, init_angles),
+                    latents=out["latents"], latents_unscaled=out["latents_unscaled"], n_unet_evals=out["n_unet_evals"])
 
     @torch.no_grad()
     def text_to_audio_clips(self, prompt: T.Union[str, T.Sequence[str], None] = None, *, converter,

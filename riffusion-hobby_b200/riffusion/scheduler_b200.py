@@ -17,7 +17,42 @@ import torch
 from riffusion import tc_ops as ops
 
 
-class PNDMSchedulerB200:
+class _Img2ImgMixin:
+    """What diffusers 0.9 `StableDiffusionImg2ImgPipeline` asks of its scheduler [memory; SURVEY Appendix D]: the
+    strength -> timestep arithmetic of `get_timesteps` and `add_noise` on fp16 latents.  Shared by both schedulers
+    (`alphas_cumprod`, `timesteps`, `config` and `set_timesteps` come from the class)."""
+
+    def img2img_timesteps(self, num_inference_steps: int, strength: float) -> T.Tuple[int, torch.Tensor, int]:
+        """`set_timesteps(n)`, then `init_timestep = min(int(n * strength) + offset, n)`,
+        `t_start = max(n - init_timestep + offset, 0)` with offset = config["steps_offset"].  Returns (t_start,
+        timesteps[t_start:], the noise timestep timesteps[t_start]).  The multistep history starts empty at t_start."""
+        if not 0.0 <= strength <= 1.0:
+            raise ValueError(f"The value of strength should in [0.0, 1.0] but is {strength}")
+        self.set_timesteps(num_inference_steps)
+        offset = self.config.get("steps_offset", 0)
+        init_timestep = min(int(num_inference_steps * strength) + offset, num_inference_steps)
+        t_start = max(num_inference_steps - init_timestep + offset, 0)
+        timesteps = self.timesteps[t_start:]
+        if len(timesteps) == 0:
+            raise ValueError(f"strength {strength} with {num_inference_steps} inference steps leaves no denoising step")
+        return t_start, timesteps, int(timesteps[0])
+
+    def add_noise_scalars(self, timestep: int) -> T.Tuple[float, float]:
+        """(sqrt(a[t]), sqrt(1 - a[t])) as fp16 values: alphas_cumprod is cast to the sample dtype before the index, and
+        `1 - a` and `** 0.5` are fp16 tensor ops (computed in fp32, rounded to fp16 once each)."""
+        a = np.float16(self.alphas_cumprod[int(timestep)].item())
+        s = np.float16(np.sqrt(np.float32(a)))
+        s1 = np.float16(np.sqrt(np.float32(np.float16(np.float32(1.0) - np.float32(a)))))
+        return float(s), float(s1)
+
+    def add_noise_fp16(self, original: torch.Tensor, noise: torch.Tensor, timestep: int) -> torch.Tensor:
+        """img2img's `add_noise` on fp16 latents: fp16(fp16(s x) + fp16(s1 noise)), every op rounded as torch rounds
+        it (rf_add_noise_f16_seq).  `add_noise` above, which riffuse uses, rounds once and stays as it is."""
+        s, s1 = self.add_noise_scalars(timestep)
+        return ops.add_noise_f16_seq(original, noise, s, s1)
+
+
+class PNDMSchedulerB200(_Img2ImgMixin):
     order = 1
 
     def __init__(self, num_train_timesteps: int = 1000, beta_start: float = 0.00085, beta_end: float = 0.012,
@@ -102,7 +137,7 @@ class PNDMSchedulerB200:
         return types.SimpleNamespace(prev_sample=self.step_cfg(pair, 0.0, int(timestep), sample))
 
 
-class DPMSolverMultistepSchedulerB200:
+class DPMSolverMultistepSchedulerB200(_Img2ImgMixin):
     """DPM-Solver++(2M): diffusers 0.9 `DPMSolverMultistepScheduler.from_config(<the PNDM config above>)`, i.e.
     algorithm_type="dpmsolver++", solver_type="midpoint", solver_order=2, lower_order_final=True, epsilon prediction, no
     thresholding [memory; SURVEY Appendix C].  The reference's default txt2img scheduler (streamlit/util.py:26-33).
@@ -112,14 +147,18 @@ class DPMSolverMultistepSchedulerB200:
     in two ping-pong buffers: step i reads the buffer step i-1 wrote and writes the other one."""
     order = 1
 
-    def __init__(self, num_train_timesteps: int = 1000, beta_start: float = 0.00085, beta_end: float = 0.012):
+    def __init__(self, num_train_timesteps: int = 1000, beta_start: float = 0.00085, beta_end: float = 0.012,
+                 steps_offset: int = 1):
         betas = torch.linspace(beta_start ** 0.5, beta_end ** 0.5, num_train_timesteps, dtype=torch.float32) ** 2
         self.alphas_cumprod = torch.cumprod(1.0 - betas, dim=0)
         self.alpha_t = torch.sqrt(self.alphas_cumprod)
         self.sigma_t = torch.sqrt(1 - self.alphas_cumprod)
         self.lambda_t = torch.log(self.alpha_t) - torch.log(self.sigma_t)
         self.num_train_timesteps = num_train_timesteps
-        self.config = {"num_train_timesteps": num_train_timesteps, "solver_order": 2, "lower_order_final": True}
+        # `from_config(<PNDM config>)` keeps the PNDM config's steps_offset = 1 as a hidden entry of the DPM config
+        # [memory; SURVEY Appendix D]; only img2img reads it, and only strength 1.0 depends on it
+        self.config = {"num_train_timesteps": num_train_timesteps, "solver_order": 2, "lower_order_final": True,
+                       "steps_offset": steps_offset}
         self.init_noise_sigma = 1.0
         self.timesteps: T.Optional[torch.Tensor] = None
         self.set_timesteps(50)

@@ -340,6 +340,54 @@ def axpby(x, noise, a, b, mask=None, z=None):
     return y
 
 
+def add_noise_f16_seq(x, noise, s, s1):
+    """diffusers 0.9 add_noise as its fp16 ops run it (rf_add_noise_f16_seq): fp16(fp16(s x) + fp16(s1 noise)), with s and
+    s1 the fp16 values of sqrt(a[t]) and sqrt(1 - a[t])."""
+    _f16(x, "x"), _f16(noise, "noise")
+    assert noise.shape == x.shape
+    x, noise = x.contiguous(), noise.contiguous()
+    y = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        _native.check(_native.lib().rf_add_noise_f16_seq(x.data_ptr(), noise.data_ptr(), float(s), float(s1), x.numel(),
+                                                         y.data_ptr(), _stream(x)))
+    return y
+
+
+def resample_u8(x_nhwc: torch.Tensor, height: int, width: int) -> torch.Tensor:
+    """Pillow-exact `Image.resize((width, height), Image.BICUBIC)` of a batch: (B, H, W, 3) uint8 -> (B, height, width, 3)
+    uint8 (rf_resample_u8)."""
+    x = _native.require_cuda(x_nhwc, "image", torch.uint8)
+    B, H, W, Cc = x.shape
+    assert Cc == 3
+    y = torch.empty((B, height, width, 3), dtype=torch.uint8, device=x.device)
+    with torch.cuda.device(x.device):
+        _native.check(_native.lib().rf_resample_u8(x.data_ptr(), B, H, W, height, width, y.data_ptr(), _stream(x)))
+    return y
+
+
+def resample_coeffs(n_in: int, n_out: int):
+    """Host tables of rf_resample_u8 along one axis: (bounds (n_out, 2) int32, taps (n_out, ksize) int32)."""
+    import numpy as np
+
+    ksize = C.c_int()
+    _native.check(_native.lib().rf_resample_coeffs(n_in, n_out, C.byref(ksize), None, None))
+    bounds = np.zeros((n_out, 2), np.int32)
+    kk = np.zeros((n_out, ksize.value), np.int32)
+    _native.check(_native.lib().rf_resample_coeffs(n_in, n_out, C.byref(ksize), bounds.ctypes.data, kk.ctypes.data))
+    return bounds, kk
+
+
+def image_u8_to_f16(x_nhwc: torch.Tensor) -> torch.Tensor:
+    """(B, H, W, 3) uint8 -> (B, 3, H, W) fp16 in [-1, 1]: img2img's preprocess (`/ 255`, `2x - 1` in fp32) + `.half()`."""
+    x = _native.require_cuda(x_nhwc, "image", torch.uint8)
+    B, H, W, Cc = x.shape
+    assert Cc == 3
+    y = torch.empty((B, 3, H, W), dtype=torch.float16, device=x.device)
+    with torch.cuda.device(x.device):
+        _native.check(_native.lib().rf_image_u8_to_f16(x.data_ptr(), B, H, W, y.data_ptr(), _stream(x)))
+    return y
+
+
 def conv1x1_small(x_nchw: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, in_scale: float = 1.0) -> torch.Tensor:
     """(B, Cin<=8, H, W) NCHW -> (B, Cout<=8, H, W); w: (Cout, Cin) fp16."""
     _f16(x_nchw, "x")
